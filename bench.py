@@ -315,6 +315,47 @@ class PairBatch:
         return np.frombuffer(self.out["results"].cpu().numpy().tobytes(), capi.PAIR_RESULT_DTYPE)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes path/<name>.npy for each array: 0/1 flags as float32, everything else as float64.  Above DUMP_BYTES in all, every
+    array keeps the same seeded sample of its rows (the same rows for the same length), so two runs with the same arguments
+    stay comparable entry for entry.  Every value written is finite: a value that is not is refused."""
+    arrays = {k: np.asarray(v, np.float32 if v.dtype == np.uint8 else np.float64) for k, v in arrays.items()}
+    for k, v in arrays.items():
+        if not np.isfinite(v).all():
+            raise ValueError("output %s has %d non-finite entries" % (k, int((~np.isfinite(v)).sum())))
+    keep = min(1.0, DUMP_BYTES / sum(v.nbytes for v in arrays.values()))
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        if keep < 1.0:
+            n = len(v)
+            v = v[np.sort(np.random.default_rng(0).choice(n, max(1, int(n * keep)), replace=False))]
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
+def pair_outputs(batches, capi):
+    """What fq_replan_pairs_dev hands its caller, batch after batch: per-candidate flags and costs of both sweeps, and the
+    fields of the per-corridor result records.  Where the library reports no result (include/faster_b200.h: the cost of a
+    candidate its flag marks infeasible; the cost and dt of a sweep without a winner, whose dt index is -1; R, and the safe
+    sweep's dt base, when the whole sweep has no winner) it leaves inf or nan: those entries are written as 0, the flags and
+    indices beside them say which they are."""
+    out = {k: np.concatenate([b.out[k].cpu().numpy() for b in batches])
+           for k in ("feasible_whole", "cost_whole", "feasible_safe", "cost_safe")}
+    res = np.concatenate([b.results(capi) for b in batches])
+    out.update({"result_" + f: res[f] for f in capi.PAIR_RESULT_DTYPE.names})
+    for s in ("whole", "safe"):
+        out["cost_" + s] = np.where(out["feasible_" + s] != 0, out["cost_" + s], 0.0)
+        won = res[s + "_dt_index"] >= 0
+        for f in (s + "_cost", s + "_dt"):
+            out["result_" + f] = np.where(won, res[f], 0.0)
+    whole_won = res["whole_dt_index"] >= 0
+    out["result_R"] = np.where(whole_won[:, None], res["R"], 0.0)
+    out["result_safe_dt_base"] = np.where(whole_won, res["safe_dt_base"], 0.0)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -333,7 +374,14 @@ def main():
     ap.add_argument("--contexts", type=int, default=3, help="solver contexts / streams the chains of consecutive batches rotate over")
     ap.add_argument("--quick", action="store_true", help="profiling runs: main timing only")
     ap.add_argument("--no-memo", action="store_true", help="A/B: switch the infeasibility-certificate memo off (option cert_memo = 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed as DIR/<name>.npy "
+                                                          "(rank 0; at most 64 MB, a fixed seeded sample of larger outputs; entries without a "
+                                                          "result, as the flags and indices show, are 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -418,6 +466,8 @@ def main():
     step_ms = timed(args.steps, inner, batches)
     total_ms = float(sum(step_ms))
     res0 = batches[0].results(capi)
+    if args.dump_outputs and rank == 0:                      # the batches the last step's passes wrote, before later legs reuse them
+        dump_outputs(args.dump_outputs, pair_outputs(batches[:min(inner, len(batches))], capi))
 
     # ---- strong scaling: the SAME 64 corridors x 1024 pairs split over the ranks (cfg4 as written: 65 536 over 8 GPUs)
     strong = None
@@ -886,6 +936,9 @@ def bench_single(args, name, torch, capi, dev, local, world, rank, barrier, main
             launch()
         ev[i][1].record(st)
     barrier()
+    if main_line and args.dump_outputs and rank == 0:
+        f = feas.cpu().numpy()
+        dump_outputs(args.dump_outputs, {"feasible": f, "cost": np.where(f != 0, cost.cpu().numpy(), 0.0)})   # as pair_outputs
     sms = [x.elapsed_time(y) for x, y in ev]
     total_ms = float(sum(sms))
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)

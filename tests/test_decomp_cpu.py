@@ -1,16 +1,38 @@
 """Host-side convex decomposition (fq_ellipsoid_decomp, faster_b200/csrc/fq_decomp.cpp) against
-  * the REFERENCE'S OWN CODE: DecompUtil's EllipsoidDecomp3D compiled unmodified from /root/reference (oracle/Makefile ->
+  * the REFERENCE'S OWN CODE: DecompUtil's EllipsoidDecomp3D compiled unmodified from the original project (oracle/Makefile ->
     oracle/_ref/libdecomp_ref.so; oracle/stub_eigen supplies the small-matrix arithmetic Eigen would), driven like
-    JPS_Manager::cvxEllipsoidDecomp (oracle/decomp_ref_wrap.cpp) -- the pinned oracle of this path;
+    JPS_Manager::cvxEllipsoidDecomp (oracle/decomp_ref_wrap.cpp) -- the pinned oracle of this path.  What it returned on the
+    inputs below is stored in tests/golden/reference_decomp.npz (tools/make_reference_goldens.py);
   * the numpy restatement of the same (oracle/decomp_oracle.py), itself checked against the compiled reference here, in the
     reference's row order."""
+import functools
+import os
+
 import numpy as np
 import pytest
 
 from faster_b200 import capi, corridor as cr
-from oracle import decomp_oracle as do, decomp_ref as dref
+from oracle import decomp_oracle as do
 
-needs_ref = pytest.mark.skipif(not dref.available(), reason="oracle/_ref/libdecomp_ref.so is built where /root/reference exists")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_decomp.npz")
+DEMO_PATH = np.array([[5, 11.5, 0.5], [13, 11.5, 3.0], [14, 10.5, 1.5], [14, 5, 2.5]], float)        # path3d.txt
+EDGE_CASES = [
+    (np.array([[0.0, 0.0, 1.0], [1.2, 0.3, 1.1]]), np.zeros((0, 3)), 0.42),
+    (np.array([[0.0, 0.0, 0.5], [0.0, 0.0, 1.6]]), np.array([[1.0, 0.2, 1.0], [-0.8, -0.9, 0.7], [2.0, 0.0, 1.0], [0.3, 1.1, 1.4], [5.0, 5.0, 5.0]]), 0.2),
+    (np.array([[0.0, 0.0, 1.0], [1.0, 0.0, 1.0]]), np.array([[2.5, 0.0, 1.0], [-1.5, 0.0, 1.0], [0.5, 2.0, 1.0], [0.5, -2.0, 1.0], [0.5, 0.0, 2.0]]), 0.0),
+    (np.array([[0.0, 0.0, 1.0], [1.0, 1.0, 1.2]]), np.array([[0.4, 1.3, 1.0]] * 3 + [[1.2, -0.4, 1.1]] * 2), 0.1),
+]
+
+
+@functools.lru_cache(maxsize=None)
+def reference(key):
+    """The reference's polytopes stored under `key`, one list of (A, b) per call, in call order."""
+    with np.load(GOLDEN) as z:
+        Ab, rows, polys = z[key + ".Ab"], z[key + ".rows"], z[key + ".polys"]
+    ends = np.cumsum(rows)
+    flat = [(Ab[e - n:e, :3], Ab[e - n:e, 3]) for n, e in zip(rows, ends)]
+    cuts = np.concatenate([[0], np.cumsum(polys)])
+    return [flat[a:b] for a, b in zip(cuts[:-1], cuts[1:])]
 
 
 def _same(polys_a, polys_b, tol=1e-9):
@@ -139,16 +161,16 @@ def _clouds(seed, n):
             yield path, obs, float(rng.choice([0.0, 0.2, 0.42]))
 
 
-@needs_ref
 def test_product_matches_the_reference_code(built_lib):
     """fq_ellipsoid_decomp against DecompUtil itself (compiled from the reference tree): the same faces to 1e-9, the six
     bounding-box faces and the ground face last and in the reference's order.  The two obstacle points the final ellipsoid
     touches are at distance 1 from it up to rounding, so the reference's first two faces may come out in either order
     (it inverts C numerically, the product keeps C^-1 in closed form): obstacle faces are compared as sets."""
     n_poly = n_rows = in_order = 0
-    for path, obs, r in _clouds(1, 45):
+    clouds = list(_clouds(1, 45))
+    assert len(clouds) == len(reference("product"))
+    for (path, obs, r), ref in zip(clouds, reference("product")):
         ours = capi.ellipsoid_decomp(path, obs, (2.0, 2.0, 1.0), r, 0.0)
-        ref = dref.cvx_ellipsoid_decomp(path, obs, (2.0, 2.0, 1.0), r, 0.0)
         _same(ours, ref)
         for (A1, b1), (A2, b2) in zip(ours, ref):
             n_poly += 1
@@ -158,15 +180,15 @@ def test_product_matches_the_reference_code(built_lib):
     assert in_order >= 0.7 * n_poly                     # and most polytopes agree row by row as well
 
 
-@needs_ref
 def test_numpy_restatement_matches_the_reference_code():
-    """oracle/decomp_oracle.py (the portable checker the other tests of this file use; the compiled reference does not exist
-    where /root/reference is absent) against the compiled reference: the same faces; and row by row in most polytopes (it
-    inverts C numerically like the reference; regularly sampled cylinders still produce exact distance ties)."""
+    """oracle/decomp_oracle.py (the checker the other tests of this file use on inputs without stored reference outputs)
+    against the compiled reference: the same faces; and row by row in most polytopes (it inverts C numerically like the
+    reference; regularly sampled cylinders still produce exact distance ties)."""
     n_poly = in_order = 0
-    for path, obs, r in _clouds(2, 30):
+    clouds = list(_clouds(2, 30))
+    assert len(clouds) == len(reference("restatement"))
+    for (path, obs, r), ref in zip(clouds, reference("restatement")):
         mine = do.cvx_ellipsoid_decomp(path, obs, (2.0, 2.0, 1.0), r, 0.0)
-        ref = dref.cvx_ellipsoid_decomp(path, obs, (2.0, 2.0, 1.0), r, 0.0)
         _same(mine, ref)
         for (A1, b1), (A2, b2) in zip(mine, ref):
             n_poly += 1
@@ -174,28 +196,20 @@ def test_numpy_restatement_matches_the_reference_code():
     assert n_poly >= 40 and in_order >= 0.8 * n_poly, (n_poly, in_order)
 
 
-@needs_ref
 def test_reference_code_reproduces_the_demo_polytopes_bbox_rows(demo_corridor):
     """The compiled reference on the demo's own path (decomp_test_node/data/path3d.txt, local bbox (1, 2, 1)) reproduces the
     six bounding-box rows of the polytopes printed in faster/other/gurobi_continuous.cpp:318-401 -- the wrapper and the Eigen
     stand-in drive the reference's code the way the reference's demo did."""
-    path = np.array([[5, 11.5, 0.5], [13, 11.5, 3.0], [14, 10.5, 1.5], [14, 5, 2.5]], float)
-    ref = dref.cvx_ellipsoid_decomp(path, np.zeros((0, 3)), (1.0, 2.0, 1.0), 0.0, -100.0)
+    ref = reference("demo")[0]
     for k, (A, b) in enumerate(demo_corridor["polys"]):
         Ar, br = ref[k]
         assert Ar.shape[0] == 7
         assert np.abs(A[-6:] - Ar[:6]).max() < 5e-5 and np.abs(b[-6:] - br[:6]).max() < 5e-5
 
 
-@needs_ref
 def test_reference_edge_cases_agree(built_lib):
     """No obstacles; a vertical segment (dir_h degenerates, line_segment.h:64-70); points exactly on a bounding-box face;
     a point on the segment's axis beyond its ends; duplicate points."""
-    cases = [
-        (np.array([[0.0, 0.0, 1.0], [1.2, 0.3, 1.1]]), np.zeros((0, 3)), 0.42),
-        (np.array([[0.0, 0.0, 0.5], [0.0, 0.0, 1.6]]), np.array([[1.0, 0.2, 1.0], [-0.8, -0.9, 0.7], [2.0, 0.0, 1.0], [0.3, 1.1, 1.4], [5.0, 5.0, 5.0]]), 0.2),
-        (np.array([[0.0, 0.0, 1.0], [1.0, 0.0, 1.0]]), np.array([[2.5, 0.0, 1.0], [-1.5, 0.0, 1.0], [0.5, 2.0, 1.0], [0.5, -2.0, 1.0], [0.5, 0.0, 2.0]]), 0.0),
-        (np.array([[0.0, 0.0, 1.0], [1.0, 1.0, 1.2]]), np.array([[0.4, 1.3, 1.0]] * 3 + [[1.2, -0.4, 1.1]] * 2), 0.1),
-    ]
-    for path, obs, r in cases:
-        _same(capi.ellipsoid_decomp(path, obs, inflate=r), dref.cvx_ellipsoid_decomp(path, obs, inflate=r))
+    assert len(reference("edge")) == len(EDGE_CASES)
+    for (path, obs, r), ref in zip(EDGE_CASES, reference("edge")):
+        _same(capi.ellipsoid_decomp(path, obs, inflate=r), ref)

@@ -1,14 +1,30 @@
-"""Host-side path search (fq_jps3d_plan*, faster_b200/csrc/fq_jps.cpp) against the REFERENCE's own graph search compiled
-from /root/reference (oracle/_ref/libjps_ref.so, built by oracle/Makefile with a stub for boost::heap).  Where the
-reference library is absent (no /root/reference and no prebuilt file) the comparisons fall back to plain A* of the
-product itself, which the reference run here has pinned to be cost-equal."""
+"""Host-side path search (fq_jps3d_plan*, faster_b200/csrc/fq_jps.cpp) against the REFERENCE's own graph search and planner
+layer compiled from the original project (oracle/_ref/libjps_ref.so and libjpsplan_ref.so, built by oracle/Makefile with
+stand-ins for boost::heap, Eigen, ROS and PCL).  What they returned on the inputs below is stored in
+tests/golden/reference_jps.npz (tools/make_reference_goldens.py)."""
+import functools
+import os
+
 import numpy as np
 import pytest
 
-from faster_b200 import capi, corridor as cr
-from oracle import jps_ref
+from faster_b200 import capi
 
-HAVE_REF = jps_ref.available()
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_jps.npz")
+RES, ORIGIN = 0.25, np.array([-5.0, -5.0, 0.0])
+
+
+@functools.lru_cache(maxsize=None)
+def reference(key):
+    with np.load(GOLDEN) as z:
+        return z[key]
+
+
+def reference_paths(key):
+    """The list of (n, 3) paths stored under `key` (rows of all paths, and each path's length)."""
+    pts, n = reference(key + ".points"), reference(key + ".n")
+    ends = np.cumsum(n)
+    return [pts[e - k:e] for k, e in zip(n, ends)]
 
 
 def _forest_grid(seed, dims=(40, 40, 12), res=0.25, n_trees=28):
@@ -50,11 +66,47 @@ def _check_path(g, path, cost):
     assert abs(total - cost) <= 1e-9 * max(1.0, cost)
 
 
+def map_queries(seed):
+    """The random map of test_costs_equal_the_reference_on_random_maps and its 12 (start, goal) pairs."""
+    g = _forest_grid(seed)
+    rng = np.random.default_rng(100 + seed)
+    return g, [(_free_cell(g, rng), _free_cell(g, rng)) for _ in range(12)]
+
+
+def hole_map():
+    """A wall splits the map; one hole in it."""
+    g = np.zeros((6, 12, 12), np.int8)
+    g[:, :, 6] = 100
+    g[2, 5, 6] = 0
+    return g
+
+
+def world_queries():
+    """(grid, world start, world goal) of test_world_plan_equals_the_reference_planner: 40 forest maps, then the refusals (an
+    occupied start, an occupied goal, a walled-in goal)."""
+    out = []
+    for seed in range(40):
+        g = _forest_grid(50 + seed)
+        rng = np.random.default_rng(seed)
+        s, t = _free_cell(g, rng), _free_cell(g, rng)
+        ws = (np.array(s) + 0.5) * RES + ORIGIN + rng.uniform(-0.1, 0.1, 3)
+        wt = (np.array(t) + 0.5) * RES + ORIGIN + rng.uniform(-0.1, 0.1, 3)
+        out.append((g, ws, wt))
+    g = _forest_grid(7)
+    occ = np.argwhere(g == 100)[0][::-1]
+    free = np.array(_free_cell(g, np.random.default_rng(1)))
+    w_occ, w_free = (occ + 0.5) * RES + ORIGIN, (free + 0.5) * RES + ORIGIN
+    out += [(g, w_occ, w_free), (g, w_free, w_occ)]
+    g2 = np.zeros((6, 12, 12), np.int8)
+    g2[:, 4:9, 4] = g2[:, 4:9, 8] = g2[:, 4, 4:9] = g2[:, 8, 4:9] = 100
+    g2[0, 4:9, 4:9] = g2[5, 4:9, 4:9] = 100                          # a closed box around the goal
+    out.append((g2, (np.array([1, 1, 2]) + 0.5) * RES + ORIGIN, (np.array([6, 6, 2]) + 0.5) * RES + ORIGIN))
+    return out
+
+
 def test_pruning_rules_equal_the_reference_tables(built_lib):
-    if not HAVE_REF:
-        pytest.skip("reference library not built here")
     ns, f1, f2, cnt = capi.jps3d_rules()
-    rn, rf1, rf2 = jps_ref.tables()
+    rn, rf1, rf2 = reference("tables.ns"), reference("tables.f1"), reference("tables.f2")
     nsz = {0: (26, 0), 1: (1, 8), 2: (3, 12), 3: (7, 12)}          # graph_search.h:123-135
     distinct = {1: 8, 2: 8, 3: 6}                                     # blockers hasForced() looks at (:420-470)
     for dz in (-1, 0, 1):
@@ -74,18 +126,14 @@ def test_pruning_rules_equal_the_reference_tables(built_lib):
 
 @pytest.mark.parametrize("seed", range(8))
 def test_costs_equal_the_reference_on_random_maps(built_lib, seed):
-    g = _forest_grid(seed)
-    rng = np.random.default_rng(100 + seed)
+    g, queries = map_queries(seed)
+    ref = reference("maps")[seed]                          # per query: JPS found, JPS cost, A* found, A* cost
     solved = 0
-    for _ in range(12):
-        s, t = _free_cell(g, rng), _free_cell(g, rng)
+    for (s, t), (rj, rcj, ra, rca) in zip(queries, ref):
         pj, cj, ej = capi.jps3d_plan(g, s, t, True)
         pa, ca, ea = capi.jps3d_plan(g, s, t, False)
         assert (len(pj) > 0) == (len(pa) > 0)
-        if HAVE_REF:
-            rj, rcj, _ = jps_ref.plan(g, s, t, True)
-            ra, rca, _ = jps_ref.plan(g, s, t, False)
-            assert (len(rj) > 0) == (len(pj) > 0) and (len(ra) > 0) == (len(pa) > 0)
+        assert bool(rj) == (len(pj) > 0) and bool(ra) == (len(pa) > 0)
         if len(pj) == 0:
             continue
         solved += 1
@@ -94,8 +142,7 @@ def test_costs_equal_the_reference_on_random_maps(built_lib, seed):
         _check_path(g, pj, cj)
         _check_path(g, pa, ca)
         assert ej <= ea                                   # jump points: never more expansions than A*
-        if HAVE_REF:
-            assert abs(cj - rcj) <= 1e-9 * rcj and abs(ca - rca) <= 1e-9 * rca
+        assert abs(cj - rcj) <= 1e-9 * rcj and abs(ca - rca) <= 1e-9 * rca
     assert solved >= 6
 
 
@@ -104,12 +151,11 @@ def test_unreachable_blocked_and_trivial(built_lib):
     g[:, :, 6] = 100                                      # a wall splits the map
     p, c, _ = capi.jps3d_plan(g, (1, 1, 1), (10, 10, 4), True)
     assert len(p) == 0 and np.isinf(c)
-    g[2, 5, 6] = 0                                        # one hole
+    g = hole_map()
     p, c, _ = capi.jps3d_plan(g, (1, 1, 1), (10, 10, 4), True)
     pa, ca, _ = capi.jps3d_plan(g, (1, 1, 1), (10, 10, 4), False)
     assert len(p) > 0 and abs(c - ca) < 1e-9 and any(tuple(q) == (6, 5, 2) for q in pa)
-    if HAVE_REF:
-        assert abs(jps_ref.plan(g, (1, 1, 1), (10, 10, 4), True)[1] - c) < 1e-9
+    assert abs(reference("hole_cost") - c) < 1e-9
     assert len(capi.jps3d_plan(g, (6, 0, 0), (1, 1, 1), True)[0]) == 0          # start occupied
     assert len(capi.jps3d_plan(g, (1, 1, 1), (40, 1, 1), True)[0]) == 0         # goal outside
     p, c, _ = capi.jps3d_plan(g, (3, 3, 3), (3, 3, 3), True)                    # start == goal
@@ -150,23 +196,20 @@ def test_world_plan_post_processing(built_lib):
     assert n_ok >= 3
 
 
-@pytest.mark.skipif(not jps_ref.planner_available(), reason="oracle/_ref/libjpsplan_ref.so is built where /root/reference exists")
 def test_world_plan_equals_the_reference_planner(built_lib):
-    """fq_jps3d_plan_world against the REFERENCE's own planner layer compiled from /root/reference (JPSPlanner<3>::plan over
+    """fq_jps3d_plan_world against the REFERENCE's own planner layer compiled from the original project (JPSPlanner<3>::plan over
     MapUtil<3>: floatToInt / intToFloat, graph search, removeLinePts, removeCornerPts forwards and backwards with the
     ray-traced line of sight -- jps_planner.cpp:196-295, map_util.h:334-383): the same way points, bit for bit, with JPS and
     with plain A*; the same refusals (start or goal not free, no path)."""
-    res, origin = 0.25, np.array([-5.0, -5.0, 0.0])
+    res, origin = RES, ORIGIN
+    queries = world_queries()
+    refs = list(zip(reference_paths("world.path"), reference_paths("world.raw"), reference("world.status")))
+    assert len(refs) == 2 * len(queries)                  # JPS, then A*, per query
     n_paths = n_simplified = 0
-    for seed in range(40):
-        g = _forest_grid(50 + seed)
-        rng = np.random.default_rng(seed)
-        s, t = _free_cell(g, rng), _free_cell(g, rng)
-        ws = (np.array(s) + 0.5) * res + origin + rng.uniform(-0.1, 0.1, 3)
-        wt = (np.array(t) + 0.5) * res + origin + rng.uniform(-0.1, 0.1, 3)
-        for use_jps in (True, False):
+    for seed, (g, ws, wt) in enumerate(queries[:40]):
+        for k, use_jps in enumerate((True, False)):
             ours, raw_len = capi.jps3d_plan_world(g, origin, res, ws, wt, use_jps)
-            ref, raw, status = jps_ref.plan_world(g, origin, res, ws, wt, use_jps)
+            ref, raw, status = refs[2 * seed + k]
             assert len(ours) == len(ref), (seed, use_jps, status)
             if len(ref):
                 assert np.array_equal(ours, ref), (seed, use_jps, np.abs(ours - ref).max())
@@ -174,19 +217,8 @@ def test_world_plan_equals_the_reference_planner(built_lib):
                 n_paths += 1
                 n_simplified += len(ref) < len(raw)
     assert n_paths >= 60 and n_simplified >= 40
-    # refusals: an occupied start, an unknown goal, a walled-in goal
-    g = _forest_grid(7)
-    occ = np.argwhere(g == 100)[0][::-1]
-    free = np.array(_free_cell(g, np.random.default_rng(1)))
-    w_occ, w_free = (occ + 0.5) * res + origin, (free + 0.5) * res + origin
-    for a, b in ((w_occ, w_free), (w_free, w_occ)):
+    # refusals: an occupied start, an occupied goal, a walled-in goal (JPS)
+    for q, (g, a, b) in enumerate(queries[40:]):
         ours, _ = capi.jps3d_plan_world(g, origin, res, a, b, True)
-        ref, _, status = jps_ref.plan_world(g, origin, res, a, b, True)
-        assert len(ours) == 0 and len(ref) == 0 and status in (1, 2)
-    g2 = np.zeros((6, 12, 12), np.int8)
-    g2[:, 4:9, 4] = g2[:, 4:9, 8] = g2[:, 4, 4:9] = g2[:, 8, 4:9] = 100
-    g2[0, 4:9, 4:9] = g2[5, 4:9, 4:9] = 100                          # a closed box around the goal
-    a, b = (np.array([1, 1, 2]) + 0.5) * res + origin, (np.array([6, 6, 2]) + 0.5) * res + origin
-    ours, _ = capi.jps3d_plan_world(g2, origin, res, a, b, True)
-    ref, _, status = jps_ref.plan_world(g2, origin, res, a, b, True)
-    assert len(ours) == 0 and len(ref) == 0 and status == -1
+        ref, _, status = refs[2 * (40 + q)]
+        assert len(ours) == 0 and len(ref) == 0 and status in ((1, 2) if q < 2 else (-1,))
